@@ -18,6 +18,8 @@ Contract (see the task statement): `python bench.py --gpus N --steps K --warmup 
     thread sweep), on bounded samples of GPU batch 0.
   * --impl reference: the oracle arm timed alone (rank 0 only under torchrun) on the first units of the SAME batch.
   * parity_sample: after the timed region, units of every resident batch are re-run through the oracle and compared.
+  * --dump-outputs DIR: what the last timed step computed (rank 0's states, covariances, result records) as DIR/*.npy;
+    the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 L2 hygiene: three different 1000-unit batches (3 x ~87 MB > 126 MB L2) are resident and used round-robin, so
 no step finds its inputs in L2.
 """
@@ -219,6 +221,24 @@ def jacobian_bytes(batch):
     return 76 * ns + 56 * nc + 384 * batch.n
 
 
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, states, covs, res, max_bytes=DUMP_MAX_BYTES):
+    """Write what lins_gpu_batch_download hands the caller of one step (posterior states, exit covariances and the fields
+    of the 64-B result records) as out_dir/<name>.npy in float64, so that two builds can be compared output for output.
+    Above max_bytes a fixed, seeded sample of the units is written (in unit order; scan_id names each one)."""
+    arrays = {"state": states, "cov": covs, "scan_id": res["scan_id"], "iters": res["iters"], "flags": res["flags"], "pose": res["pose"]}
+    n = len(res)
+    row_bytes = sum(8 * (np.asarray(a).size // max(1, n)) for a in arrays.values())
+    keep = (max_bytes - 1024 * len(arrays)) // row_bytes  # (room for the .npy headers)
+    idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if n > keep else np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64)[idx])
+    return sorted(arrays)
+
+
 def reference_arm(args, rank, world):
     """--impl reference: the CPU oracle (port of the reference path; the reference itself needs ROS/PCL/Eigen and
     cannot be built here), reference-faithful M x M gain, scan-parallel over the host cores (best of a thread sweep),
@@ -264,7 +284,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scans", type=int, default=SCANS_PER_GPU, help="units per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none to write")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -382,6 +405,9 @@ def main():
     else:
         total_iters, total_launches = float(my_iters), launches
     value = total_iters / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:  # (before the e2e legs below re-use these contexts)
+        so, co, res, _ = ctxs[(args.steps - 1) % NB].batch_download(states=True, covs=True)
+        dump_outputs(args.dump_outputs, so, co, res)
 
     # ---- end to end through the C-ABI with host buffers (pack + H2D + kernel + D2H timed) ------------------------
     # The user-facing call is lins_gpu_ieskf_batch(ctx, host batch) -> host results (synchronous: pack, H2D, the

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -29,6 +31,28 @@ def test_host_memory_policy_is_harmless():
     on = b.host_memory_policy(True)
     off = b.host_memory_policy(False)
     assert isinstance(on, str) and isinstance(off, str)  # one node / refused / interleaved: never raises
+
+
+def test_dump_outputs_writes_float64_within_the_cap(tmp_path):
+    b = _bench()
+    defs = importlib.import_module("lins---lidar-inertial-slam_b200.ctypes_defs")
+    n = 500
+    res = np.zeros(n, dtype=defs.SCAN_RESULT_DTYPE)
+    res["scan_id"] = np.arange(n); res["iters"] = 7; res["flags"] = 1; res["pose"] = np.arange(7 * n).reshape(n, 7)
+    states, covs = np.random.default_rng(1).standard_normal((n, defs.STATE_DIM)), np.ones((n, defs.COV_SIZE))
+    full = b.dump_outputs(str(tmp_path / "full"), states, covs, res)
+    assert full == ["cov", "flags", "iters", "pose", "scan_id", "state"]
+    got = {k: np.load(tmp_path / "full" / f"{k}.npy") for k in full}
+    assert all(a.dtype == np.float64 and len(a) == n for a in got.values())
+    assert np.array_equal(got["state"], states) and np.array_equal(got["pose"], res["pose"])
+    cap = 300_000  # < n rows: a seeded sample of the units, the same one every time
+    for d in ("s1", "s2"):
+        b.dump_outputs(str(tmp_path / d), states, covs, res, max_bytes=cap)
+    assert sum(os.path.getsize(p) for p in (tmp_path / "s1").iterdir()) <= cap
+    ids = np.load(tmp_path / "s1" / "scan_id.npy")
+    assert 0 < len(ids) < n and np.all(np.diff(ids) > 0)
+    assert np.array_equal(ids, np.load(tmp_path / "s2" / "scan_id.npy"))
+    assert np.array_equal(np.load(tmp_path / "s1" / "state.npy"), states[ids.astype(int)])
 
 
 def test_reference_arm_prints_one_json_line():
